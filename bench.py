@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          the CUDA path (this repo)
   python bench.py --impl reference --gpus N ...           the reference's CPU algorithm (oracle port) on the host cores
+  python bench.py --gpus 1 ... --dump-outputs DIR         also write the last timed step's octree as DIR/*.npy (see dump_outputs)
 
 A step = one build_octree over one batch of synthetic points (BASELINE.json config 2: Gaussian clusters in a 1024 m cube,
 resolution 1024/2^20 -> depth 20, 1e9 points per GPU).  At N > 1 every rank owns the same number of points of one global index
@@ -397,6 +398,47 @@ def full_size_check(tree, D, torch, dist, world, n, dev):
     return {"ok": got == want, "points": got[0], "expected_points": NT, "sum_idx_ok": got[1] == want[1], "sum_idx_sq_ok": got[2] == want[2]}
 
 
+DUMP_BYTES = 64_000_000
+DUMP_SEED = 20240917
+
+
+def dump_outputs(tree, directory):
+    """What the timed build hands its caller, for output-for-output comparison of two builds on the same seeded input:
+    the whole node table (nodes.npy, one row per node in (id_high, id_low) order: level, the two 64-bit id words as 32-bit
+    halves, num_points, position encoding, cube min xyz, edge) and, for a seeded sample of whole nodes that fits the 64 MB
+    budget, every point of those nodes in slot order (sample_*.npy: node row, position code as stored, colour, source index)."""
+    import numpy as np
+
+    m = tree.meta
+    rows = np.lexsort((m["id_low"], m["id_high"]))
+    half = lambda v: [(v >> np.uint64(32)).astype(np.float64), (v & np.uint64(0xFFFFFFFF)).astype(np.float64)]
+    nodes = np.stack([m["level"][rows].astype(np.float64)] + half(m["id_high"][rows]) + half(m["id_low"][rows])
+                     + [m["num_points"][rows].astype(np.float64), m["enc"][rows].astype(np.float64)]
+                     + [m["cube"][rows, k] for k in range(4)], 1)
+    per_point = 8 + 3 * 8 + 3 * 4 + 8
+    budget = (DUMP_BYTES - nodes.nbytes) // per_point
+    picked, total = [], 0
+    for r in np.random.default_rng(DUMP_SEED).permutation(len(rows)):
+        k = int(m["num_points"][rows[r]])
+        if k and total + k <= budget:
+            picked.append(int(r))
+            total += k
+    node_of, code, rgb, src = [], [], [], []
+    for r in sorted(picked):
+        xyz, c, _, s = tree.node_data_at(int(rows[r]))
+        dt = {1: "<u1", 2: "<u2", 3: "<f4", 4: "<f8"}[int(m["enc"][rows[r]])]
+        code.append(np.frombuffer(xyz.tobytes(), dt).reshape(-1, 3).astype(np.float64))
+        rgb.append(c.reshape(-1, 3).astype(np.float32))
+        src.append(s.astype(np.float64))
+        node_of.append(np.full(len(s), r, np.float64))
+    out = {"nodes": nodes, "sample_node": np.concatenate(node_of or [np.zeros(0)]), "sample_position_code": np.concatenate(code or [np.zeros((0, 3))]),
+           "sample_rgb": np.concatenate(rgb or [np.zeros((0, 3), np.float32)]), "sample_source_index": np.concatenate(src or [np.zeros(0)])}
+    assert sum(a.nbytes for a in out.values()) <= DUMP_BYTES
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -490,6 +532,8 @@ def run_ours(args):
     sampler.window(t_region0, time.time())
     clocks = sampler.stop() if rank == 0 else None
     launches = ctx.kernel_launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(last, args.dump_outputs)
     tm = torch.tensor([dev_ms, wall_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(tm, op=dist.ReduceOp.MAX)
@@ -787,7 +831,12 @@ def main():
     ap.add_argument("--ref-points", type=float, default=1e8, help="points of the bounded sample each --impl reference step builds")
     ap.add_argument("--no-extras", action="store_true", help="profiling runs: only the timed build steps (no roofline / query / e2e / CPU legs)")
     ap.add_argument("--roofline-only", action="store_true", help="development runs: timed steps + per-kernel roofline, none of the other legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's octree (node table + a seeded sample of its points) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the single-GPU build (--impl ours, one process)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

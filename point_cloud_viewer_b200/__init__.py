@@ -450,9 +450,11 @@ class Octree:
         return xyz, rgb, inten, src
 
     def free(self):
-        if self.h:
+        # pcv_octree_free works through the owning pcv_ctx, so it must not run once that context is destroyed (an octree that
+        # outlives Context.close(), e.g. one collected at interpreter exit)
+        if self.h and self.ctx.h:
             N.lib().pcv_octree_free(self.h)
-            self.h = None
+        self.h = None
 
     def __del__(self):
         try:
@@ -649,9 +651,9 @@ class S2Cloud:
         N.check(N.lib().pcv_s2_cells(self.h, _p(self.cell_ids), _p(self.cell_counts)))
 
     def free(self):
-        if self.h:
+        if self.h and self.ctx.h:  # as Octree.free: pcv_s2_free needs the owning pcv_ctx alive
             N.lib().pcv_s2_free(self.h)
-            self.h = None
+        self.h = None
 
     def write_dir(self, directory):
         """<token>.xyz / .rgb / .intensity per cell + meta.pb, as S2Splitter<RawNodeWriter> leaves them."""
