@@ -154,10 +154,23 @@ int pcv_visible_nodes(const pcv_octree* o, const double clip_from_world[16], uin
  * into batches of exactly batch_size points (last one short), on the caller's thread. */
 int pcv_query_points(const pcv_octree* o, const pcv_location* loc, const pcv_interval* filters, uint32_t nfilt,
                      uint64_t batch_size, pcv_batch_cb cb, void* user);
+/* Survivors of pcv_query_batch_device, written to caller-owned device buffers of `cap` points.  Inside one location
+ * every point appears at most once; the order across and inside locations is unspecified.  Survivors beyond `cap`
+ * are counted in counts_out but not stored. */
+typedef struct pcv_query_out {
+    double* xyz;         /* cap * 3, decoded positions                                           */
+    uint8_t* rgb;        /* cap * 3                                                              */
+    float* intensity;    /* cap, or NULL (ignored when the octree has no intensity)              */
+    uint32_t* src_index; /* cap: the u32 source index the octree holds                           */
+    uint32_t* loc;       /* cap, or NULL: index into locs[] of each survivor                     */
+    uint64_t cap;
+    uint64_t stored;     /* out: survivors written, = min(cap, sum of counts_out)                */
+} pcv_query_out;
 /* Throughput form: nloc locations in one call; survivors stay compacted in HBM.  counts_out[i] =
- * survivors of location i, tested_out[i] = points decoded + tested for location i. */
+ * survivors of location i, tested_out[i] = points decoded + tested for location i.  out == NULL: the
+ * survivors go to scratch buffers (capacity min(points tested, 192 Mi)) that are freed before the call returns. */
 int pcv_query_batch_device(const pcv_octree* o, const pcv_location* locs, uint32_t nloc, const pcv_interval* filters,
-                           uint32_t nfilt, uint64_t* counts_out, uint64_t* tested_out);
+                           uint32_t nfilt, uint64_t* counts_out, uint64_t* tested_out, pcv_query_out* out);
 
 /* Timing / traffic of the last pcv_query_batch_device call on the context (CUDA events on the context's stream). */
 typedef struct pcv_query_stats {

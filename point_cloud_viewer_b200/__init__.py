@@ -555,13 +555,37 @@ class Octree:
         N.check(rc)
         return got
 
-    def query_batch_device(self, locs, filters=()):
+    def query_batch_device(self, locs, filters=(), points=False, cap=None):
+        """Per-location survivor and tested counts of a batch of locations.  points=True also returns the survivors, copied to
+        the host: dict(loc, src (u32), xyz (n,3) f64, rgb (n,3), intensity or None, stored), in no particular order.  They land
+        in device buffers of `cap` points; cap=None sizes them to the survivor total with a first, counting call."""
         arr = (N.Location * len(locs))(*locs)
         f = np.asarray(filters, np.float64).reshape(-1)
         nf = len(f) // 2
         counts, tested = np.zeros(len(locs), np.uint64), np.zeros(len(locs), np.uint64)
-        N.check(N.lib().pcv_query_batch_device(self.h, arr, len(locs), _p(f) if nf else None, nf, _p(counts), _p(tested)))
-        return counts, tested
+        if not points:
+            N.check(N.lib().pcv_query_batch_device(self.h, arr, len(locs), _p(f) if nf else None, nf, _p(counts), _p(tested), None))
+            return counts, tested
+        if cap is None:
+            cap = int(self.query_batch_device(locs, filters)[0].sum())
+        cap = int(cap)
+        ctx, rows = self.ctx, max(cap, 1)
+        bufs = dict(xyz=ctx.device_buffer((rows, 3), "<f8"), rgb=ctx.device_buffer((rows, 3), "|u1"), src=ctx.device_buffer((rows,), "<i4"),
+                    loc=ctx.device_buffer((rows,), "<i4"))
+        if self.has_intensity:
+            bufs["intensity"] = ctx.device_buffer((rows,), "<f4")
+        try:
+            out = N.QueryOut(bufs["xyz"].ptr, bufs["rgb"].ptr, bufs["intensity"].ptr if self.has_intensity else None, bufs["src"].ptr, bufs["loc"].ptr, cap, 0)
+            N.check(N.lib().pcv_query_batch_device(self.h, arr, len(locs), _p(f) if nf else None, nf, _p(counts), _p(tested), C.byref(out)))
+            n = int(out.stored)
+            got = {k: b.tensor()[:n].cpu().numpy() for k, b in bufs.items()}  # the call has synchronised the context's stream
+        finally:
+            for b in bufs.values():
+                b.free()
+        got["src"], got["loc"] = got["src"].view(np.uint32), got["loc"].view(np.uint32)
+        got.setdefault("intensity", None)
+        got["stored"] = n
+        return counts, tested, got
 
     def last_query_stats(self):
         """Timing / traffic of the last query_batch_device call (pcv_query_stats)."""

@@ -103,6 +103,13 @@ class QueryStats(C.Structure):
                 ("tested_points", C.c_uint64), ("returned_points", C.c_uint64), ("stored_points", C.c_uint64), ("visited_pairs", C.c_uint64)]
 
 
+class QueryOut(C.Structure):
+    """pcv_query_out (include/pcv.h): caller-owned device buffers for the survivors of pcv_query_batch_device."""
+
+    _fields_ = [("xyz", C.c_void_p), ("rgb", C.c_void_p), ("intensity", C.c_void_p), ("src_index", C.c_void_p), ("loc", C.c_void_p),
+                ("cap", C.c_uint64), ("stored", C.c_uint64)]
+
+
 class XrayStats(C.Structure):
     """pcv_xray_stats (include/pcv.h)."""
 
@@ -175,7 +182,7 @@ SYMBOLS = [
     ("pcv_nodes_in_location", C.c_int, [C.c_void_p, C.POINTER(Location), C.c_void_p, C.c_uint64, _u64p]),
     ("pcv_visible_nodes", C.c_int, [C.c_void_p, _dp, C.c_void_p, C.c_uint64, _u64p]),
     ("pcv_query_points", C.c_int, [C.c_void_p, C.POINTER(Location), C.c_void_p, C.c_uint32, C.c_uint64, BATCH_CB, C.c_void_p]),
-    ("pcv_query_batch_device", C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
+    ("pcv_query_batch_device", C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(QueryOut)]),
     ("pcv_last_query_stats", C.c_int, [C.c_void_p, C.POINTER(QueryStats)]),
     ("pcv_last_xray_stats", C.c_int, [C.c_void_p, C.POINTER(XrayStats)]),
     ("pcv_xray_tile", C.c_int, [C.c_void_p, _dp, _dp, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]),

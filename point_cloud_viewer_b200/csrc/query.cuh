@@ -225,6 +225,7 @@ struct CullArgs {
     uint8_t* out_rgb;
     float* out_intensity;
     uint32_t* out_src;
+    uint32_t* out_loc;       // k_cull_fused only (may be null): the location index of every survivor
 };
 
 __device__ __forceinline__ uint64_t load_code(const uint8_t* p, int enc) {
@@ -493,6 +494,7 @@ __global__ void __launch_bounds__(256) k_pairs_to_tiles(const uint2* __restrict_
 // 256 points the block counts its survivors with ballots, reserves their output range with one atomic, stages them in shared
 // memory and copies them out as contiguous words (the order inside a round is kept; rounds land in the order they finish -
 // the batched form only promises per-location totals and the compacted set).  Survivors beyond `cap` are counted, not stored.
+// With out_loc set, every stored survivor also gets the index of its location.
 struct CullFusedArgs {
     CullArgs c;
     unsigned long long* cursor;  // output slots handed out so far
@@ -594,6 +596,7 @@ __global__ void __launch_bounds__(256) k_cull_fused(const __grid_constant__ Cull
             for (uint32_t k = threadIdx.x; k < room; k += 256) {
                 a.out_src[base + k] = st_src[k];
                 if (a.out_intensity) a.out_intensity[base + k] = st_int[k];
+                if (a.out_loc) a.out_loc[base + k] = t.loc;  // tile-uniform: no staging
             }
             __syncthreads();  // the staging arrays and wcnt are reused by the next round
         }

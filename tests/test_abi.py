@@ -29,12 +29,13 @@ def test_struct_layouts_match_header():
 
 
 def test_xray_quadtree_structs_match_the_c_compiler(tmp_path):
-    """pcv_xray_quadtree_params / _info: ctypes sizes and field offsets equal gcc's for include/pcv.h."""
+    """pcv_xray_quadtree_params / _info and pcv_query_out: ctypes sizes and field offsets equal gcc's for include/pcv.h."""
     import subprocess
 
     from point_cloud_viewer_b200 import _native as N
 
-    fields = {"pcv_xray_quadtree_params": [f for f, _ in N.XrayQuadtreeParams._fields_], "pcv_xray_quadtree_info": [f for f, _ in N.XrayQuadtreeInfo._fields_]}
+    structs = (("pcv_xray_quadtree_params", N.XrayQuadtreeParams), ("pcv_xray_quadtree_info", N.XrayQuadtreeInfo), ("pcv_query_out", N.QueryOut))
+    fields = {st: [f for f, _ in cls._fields_] for st, cls in structs}
     src = ['#include <stdio.h>', '#include <stddef.h>', '#include "pcv.h"', "int main(void) {"]
     for st, fs in fields.items():
         src.append('printf("%s %%zu" "\\n", sizeof(%s));' % (st, st))
@@ -46,7 +47,7 @@ def test_xray_quadtree_structs_match_the_c_compiler(tmp_path):
     exe = str(tmp_path / "layout")
     subprocess.check_call(["gcc", "-I", os.path.join(ROOT, "include"), "-o", exe, str(c)])
     got = dict(l.split() for l in subprocess.check_output([exe], text=True).splitlines())
-    for st, cls in (("pcv_xray_quadtree_params", N.XrayQuadtreeParams), ("pcv_xray_quadtree_info", N.XrayQuadtreeInfo)):
+    for st, cls in structs:
         assert int(got[st]) == C.sizeof(cls)
         for f, _ in cls._fields_:
             assert int(got["%s.%s" % (st, f)]) == getattr(cls, f).offset, (st, f)
